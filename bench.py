@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PAF overlaps/s, ingest -> GFA, on synthetic PAF of the shapes BASELINE.json names.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl b200|reference] [--quick]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl b200|reference] [--quick] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path over one PAF: parse -> read selection -> string graph ->
 transitive reduction -> cleaning -> unitigs (main.c:108-199 of the reference).
@@ -26,6 +26,8 @@ file order (rank r generates and holds part r), read ids are hash-sharded (owner
            reference's time on the same file.
 * host_affinity : every rank runs on the host cores NVML names for its GPU (bound before the pinned buffers are allocated).
 --impl reference prints the same line for the reference's own CPU implementation (rank 0 only).
+--dump-outputs DIR writes the unitig graph the last timed step left (what mab_export_ug / _dict / _sub hand a caller) as
+float64 .npy files, so that two builds can be compared output for output on the same seeded input.
 """
 import argparse
 import ctypes as C
@@ -241,6 +243,44 @@ def config_of(name, world):
             if world > 1 else "1 GPU"}
 
 
+DUMP_MAX_BYTES = 60 << 20   # whole dump; rows beyond an even share per array are a seeded sample (the limit is 64 MB)
+
+
+def dump_outputs(lib, ctx, out_dir):
+    """The layout the pipeline hands a caller, as float64 arrays (every value below 2^53, so exact).  Each array's column 0 is
+    the row index, so that a sampled array (a fixed, seeded sample of the rows beyond its share of DUMP_MAX_BYTES) can still be
+    compared row by row.  Tables without rows are not written."""
+    import numpy as np
+    from miniasm_b200 import capi
+    d, sub, ug = lib.mab_export_dict(ctx), lib.mab_export_sub(ctx), lib.mab_export_ug(ctx)
+    u, n_seq = ug.contents, d.contents.n_seq
+    utgs = [u.a[i] for i in range(u.n)]
+    reads = capi.np_from_ptr(sub, n_seq, capi.SUB_DT) if sub else np.zeros(n_seq, dtype=capi.SUB_DT)
+    seq_len = np.array([d.contents.seq[i].len for i in range(n_seq)], dtype=np.float64)
+    members = np.concatenate([capi.np_from_ptr(x.a, x.n, np.uint64) for x in utgs]) if utgs else np.zeros(0, np.uint64)
+    arcs = lib.read_graph(u.g)[0]
+    tables = {
+        "unitigs": np.array([[x.len_circ & 0x7fffffff, x.len_circ >> 31, x.start, x.end, x.n] for x in utgs]).reshape(-1, 5),  # length, circular, ends, reads
+        "unitig_reads": np.stack([np.repeat(np.arange(len(utgs)), [x.n for x in utgs]), members >> 32, members & 0xffffffff], 1),
+        "unitig_arcs": np.stack([arcs["ul"] >> 32, arcs["ul"] & 0xffffffff, arcs["v"], arcs["ol_del"] & 0x7fffffff, arcs["ol_del"] >> 31], 1),
+        "reads": np.stack([seq_len, reads["s_del"] & 0x7fffffff, reads["s_del"] >> 31, reads["e"]], 1),            # length, kept interval
+    }
+    tables = {k: t for k, t in tables.items() if len(t)}       # e.g. no links between unitigs: an empty array compares nothing
+    max_rows = DUMP_MAX_BYTES // (8 * sum(t.shape[1] + 1 for t in tables.values()))
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in tables.items():
+        t = t.astype(np.float64)
+        rows = np.arange(len(t))
+        if len(t) > max_rows:
+            rows = np.sort(np.random.default_rng(0).choice(len(t), max_rows, replace=False))
+        t = np.concatenate([rows[:, None].astype(np.float64), t[rows]], 1)
+        np.save(os.path.join(out_dir, f"{name}.npy"), t)
+        total += t.nbytes
+    lib.ma_ug_destroy(ug), capi.c_free(sub), lib.sd_destroy(d)
+    assert total <= 64 << 20, total
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -251,7 +291,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="skip the extra legs: full-size reference run, cold CLI wall clock, noisy workload")
     ap.add_argument("--host-gfa", action="store_true", help="e2e leg: host structs + ma_ug_print instead of the GFA text formatted on the GPU (mab_write_gfa)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the unitig graph of the last timed step to DIR/<name>.npy (float64)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     name = a.workload or BY_GPUS.get(world) or "c3_1m"
@@ -330,7 +373,7 @@ def main():
         if world > 1:
             dist.barrier()
 
-    def measure(args_str, steps, warmup, with_roofline):
+    def measure(args_str, steps, warmup, with_roofline, dump_dir=None):
         """value + e2e legs over one PAF (this rank's part of it)."""
         buf, n_bytes, n_lines, free = generate_args(args_str, rank, world)
         pinned = torch.empty(max(n_bytes, 1), dtype=torch.uint8, pin_memory=True)
@@ -385,6 +428,8 @@ def main():
             dt_ms.append((ms, lib.mab_stats(ctx).contents.ms_del_trans_kernel))
         barrier()
         wall_dev = time.perf_counter() - t_wall0
+        if dump_dir and rank == 0:                  # untimed; the graph is replicated on every rank
+            dump_outputs(lib, ctx, dump_dir)
         st = lib.mab_stats(ctx).contents
         cl = [C.c_uint32() for _ in range(4)]
         lib.mab_clean_totals(*[C.byref(x) for x in cl])
@@ -432,7 +477,7 @@ def main():
 
     sampler = ClockSampler(local_rank)
     sampler.start()
-    res = measure(wl["args"], a.steps, a.warmup, True)
+    res = measure(wl["args"], a.steps, a.warmup, True, a.dump_outputs)
     clocks = sampler.finish()
     dev_ms, e2e_s, lines_all, bytes_all = reduce_ranks(res)
 

@@ -89,10 +89,10 @@ def _model_body(rank, world, port, paf, q):
     from miniasm_b200 import capi
     from miniasm_b200.capi import HIT_DT, SUB_DT
     from miniasm_b200.pipeline import Pipeline
-    from oracle import loaders
+    from tests import reference
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
     dist.init_process_group("gloo", rank=rank, world_size=world)
-    ref = loaders.load_reference()
+    ref = reference.load()
     ref.set_verbose(0)
     data = open(paf, "rb").read()
     b, e = sharded.split_ranges(data, world)[rank]
@@ -256,9 +256,7 @@ def _model_worker(rank, world, port, paf, q):
 
 @pytest.mark.parametrize("world", [2, 3])
 def test_sharding_scheme_model(world, built, paf_dir):
-    from oracle import loaders
-    if not os.path.exists(loaders.REFERENCE_SO):
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+    from tests import reference
     paf = synth.generate("-n 3000 -s 78 -j 300 -l 8000 -L 12000", f"{paf_dir}/dist_model.paf")
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
@@ -282,4 +280,5 @@ def test_sharding_scheme_model(world, built, paf_dir):
     assert all(r[1] for r in res), res
     # the model has teeth: hits on every rank, contained reads flagged, a non-trivial graph
     assert all(r[2] > 0 and r[4] > 100 and r[5] >= r[4] and r[6] > 100 for r in res), res
+    reference.pin([r[2:] for r in res])                 # the counts the reference's compute gave every rank
     print(res)

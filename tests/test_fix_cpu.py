@@ -50,8 +50,10 @@ class Stepper:
         if got:
             ref.asg_cleanup(h)
         assert got == want, f"{name}: {got} != {want}"
-        a, s, i, f1, f2 = ref.read_graph(h)
-        b, t, j, g1, g2 = ref.read_graph(g)
+        # read back unpinned: on jittered sets the arcs a pass leaves marked can follow the order of tied arcs, which the reference's
+        # unstable sort and the port's stable one settle differently (DESIGN.md "Tie order"); the counts are pinned
+        a, s, i, f1, f2 = capi.Lib.read_graph(h)
+        b, t, j, g1, g2 = capi.Lib.read_graph(g)
         assert np.array_equal(a, b) and np.array_equal(s, t) and (f1, f2) == (g1, g2), name
         assert (i is None) == (j is None) and (i is None or np.array_equal(i, j))
         ref.asg_destroy(h)

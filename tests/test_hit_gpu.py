@@ -8,6 +8,7 @@ import pytest
 from miniasm_b200 import capi, synth
 from miniasm_b200.capi import HIT_DT, SUB_DT
 from miniasm_b200.pipeline import Pipeline, canon_arcs
+from tests import reference
 
 pytestmark = pytest.mark.gpu
 
@@ -36,8 +37,9 @@ def test_stage_i_stepwise(name, pafs, ref, prod):
     r = Pipeline(ref, pafs[name]).read()
     p = Pipeline(prod, pafs[name]).read()
     # ma_hit_read: same ids/names, same multiset of hits, same key order (ties may permute: unstable reference sort)
-    assert r.names() == p.names() and np.array_equal(r.seq_lens(), p.seq_lens())
+    assert reference.pin(r.names()) == p.names() and np.array_equal(reference.pin(r.seq_lens()), p.seq_lens())
     hr, hp = r.hits_np(), p.hits_np()
+    reference.pin(reference.hits(hr))
     assert len(hr) == len(hp) and np.array_equal(hr["qns"], hp["qns"])
     assert np.array_equal(canon_hits(hr), canon_hits(hp))
 
@@ -45,12 +47,13 @@ def test_stage_i_stepwise(name, pafs, ref, prod):
         return Pipeline(prod, pafs[name], opt=r.opt).adopt(r)
 
     def same_hits(x, y):
+        reference.pin(reference.hits(x.hits_np()))
         return x.n_hits == y.n_hits and np.array_equal(canon_mask(x.hits_np()), canon_mask(y.hits_np()))
 
     # ma_hit_sub (round 1)
     q = fresh()
     r.sub1(), q.sub1()
-    assert np.array_equal(r.sub_np(), q.sub_np())
+    assert np.array_equal(reference.pin(r.sub_np()), q.sub_np())
     q.free()
     # ma_hit_cut
     q = fresh()
@@ -61,19 +64,19 @@ def test_stage_i_stepwise(name, pafs, ref, prod):
     q = fresh()
     r.flt(), q.flt()
     assert same_hits(r, q)
-    assert r.cov.value == q.cov.value or (np.isnan(r.cov.value) and np.isnan(q.cov.value))
+    assert reference.pin(r.cov.value) == q.cov.value or (np.isnan(r.cov.value) and np.isnan(q.cov.value))
     q.free()
     # ma_hit_sub (round 2, end clip) + ma_hit_cut + ma_sub_merge
     q = fresh()
     r.sub2_cut_merge(), q.sub2_cut_merge()
-    assert np.array_equal(r.sub_np(), q.sub_np())
+    assert np.array_equal(reference.pin(r.sub_np()), q.sub_np())
     assert same_hits(r, q)
     q.free()
     # ma_hit_contained (+ dictionary squeeze)
     q = fresh()
     r.contained(), q.contained()
-    assert r.names() == q.names()
-    assert np.array_equal(r.sub_np(), q.sub_np())
+    assert reference.pin(r.names()) == q.names()
+    assert np.array_equal(reference.pin(r.sub_np()), q.sub_np())
     assert same_hits(r, q)
     q.free()
     # ma_sg_gen
@@ -114,7 +117,7 @@ def test_sub_edge_cases(ref, prod):
         pa = capi.c_malloc_copy(a)
         sr = ref.ma_hit_sub(3, 0.05, clip, len(a), pa, 16)
         sp = prod.ma_hit_sub(3, 0.05, clip, len(a), pa, 16)
-        assert np.array_equal(capi.np_from_ptr(sr, 16, SUB_DT), capi.np_from_ptr(sp, 16, SUB_DT))
+        assert np.array_equal(reference.pin(capi.np_from_ptr(sr, 16, SUB_DT)), capi.np_from_ptr(sp, 16, SUB_DT))
         capi.c_free(sr), capi.c_free(sp), capi.c_free(pa)
 
 
@@ -148,7 +151,7 @@ def test_sub_group_sizes(span, ref, prod):
         pa = capi.c_malloc_copy(a)
         sr = ref.ma_hit_sub(dp, 0.05, clip, len(a), pa, 200)
         sp = prod.ma_hit_sub(dp, 0.05, clip, len(a), pa, 200)
-        assert np.array_equal(capi.np_from_ptr(sr, 200, SUB_DT), capi.np_from_ptr(sp, 200, SUB_DT)), (dp, clip)
+        assert np.array_equal(reference.pin(capi.np_from_ptr(sr, 200, SUB_DT)), capi.np_from_ptr(sp, 200, SUB_DT)), (dp, clip)
         capi.c_free(sr), capi.c_free(sp), capi.c_free(pa)
 
 

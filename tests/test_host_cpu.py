@@ -8,6 +8,7 @@ import pytest
 from miniasm_b200 import capi, synth
 from oracle import loaders
 from miniasm_b200.pipeline import Pipeline
+from tests import reference
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -77,7 +78,6 @@ def test_sdict(built):
     prod.sd_destroy(d)
 
 
-@pytest.mark.skipif(not os.path.exists(loaders.REFERENCE_SO), reason="oracle/_ref not built")
 def test_writers_and_ug_seq_against_reference(built, ref, paf_dir):
     from tests.test_clean_gpu import _write_reads
     prod = capi.load_product()
@@ -98,7 +98,6 @@ def test_writers_and_ug_seq_against_reference(built, ref, paf_dir):
         a.free(), b.free()
 
 
-@pytest.mark.skipif(not os.path.exists(loaders.REFERENCE_SO), reason="oracle/_ref not built")
 def test_ug_seq_refuses_a_short_record(built, paf_dir):
     """asm.c:263 asserts that a record covers the interval the layout keeps; ours must not read past a shorter record either
     (a reads file that does not belong to the PAF): message + abort, in a child process."""
@@ -109,8 +108,8 @@ import sys, os
 sys.path.insert(0, {ROOT!r})
 from miniasm_b200 import capi, synth
 from miniasm_b200.pipeline import Pipeline
-from oracle import loaders
-ref = loaders.load_reference(); ref.set_verbose(0)
+from tests import reference
+ref = reference.load(); ref.set_verbose(0)
 prod = capi.load_product(); prod.set_verbose(0)
 paf = synth.generate("tiny_exact", {paf_dir!r} + "/short.paf")
 b = Pipeline(ref, paf).read().select().sg_gen().clean().ug_gen()
@@ -129,7 +128,6 @@ print("survived")
     assert "[E::ma_ug_seq]" in r.stderr and "wrong reads file" in r.stderr
 
 
-@pytest.mark.skipif(not os.path.exists(loaders.REFERENCE_SO), reason="oracle/_ref not built")
 def test_no_cont_prefilter_against_reference(built, ref, paf_dir):
     prod = capi.load_product()
     paf = synth.generate("-n 4000 -l 2000 -L 30000 -c 30 -j 100 -s 41", f"{paf_dir}/nocont.paf")
@@ -137,7 +135,7 @@ def test_no_cont_prefilter_against_reference(built, ref, paf_dir):
     b = prod.ma_hit_no_cont(paf.encode(), 2000, 100, 1000, 0.8)
     na = [a.contents.seq[i].name for i in range(a.contents.n_seq)]
     nb = [b.contents.seq[i].name for i in range(b.contents.n_seq)]
-    assert na == nb and len(na) > 10
+    assert reference.pin(na) == nb and len(na) > 10
 
 
 def test_device_parser_matches_host_reader(built, paf_dir):

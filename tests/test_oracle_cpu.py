@@ -9,8 +9,8 @@ import pytest
 from miniasm_b200 import capi, synth
 from oracle import loaders
 from miniasm_b200.pipeline import Pipeline, canon_arcs
+from tests import reference
 
-pytestmark = pytest.mark.skipif(not os.path.exists(loaders.REFERENCE_SO), reason="oracle/_ref not built (needs /root/reference)")
 SETS = ["tiny_exact", "chaos_small", "chaos", "bubbles800", "shuffled", "lowcov", "varlen300", "skew_small", "c1_ecoli_like"]
 
 
@@ -29,7 +29,8 @@ def mask(h):
 def test_port_matches_reference_stepwise(name, ref, port, paf_dir):
     paf = synth.generate(name, f"{paf_dir}/{name}.paf")
     r, p = Pipeline(ref, paf).read(), Pipeline(port, paf).read()
-    assert r.names() == p.names()
+    assert reference.pin(r.names()) == p.names()
+    reference.pin(reference.hits(r.hits_np()))
     assert np.array_equal(np.sort(mask(r.hits_np()), order=list(capi.HIT_DT.names)), np.sort(mask(p.hits_np()), order=list(capi.HIT_DT.names)))
     p.free()
     p = Pipeline(port, paf, opt=r.opt).adopt(r)      # continue from the reference's own (tie-ordered) hit array
@@ -37,7 +38,8 @@ def test_port_matches_reference_stepwise(name, ref, port, paf_dir):
         getattr(r, step)(), getattr(p, step)()
         assert r.n_hits == p.n_hits and np.array_equal(mask(r.hits_np()), mask(p.hits_np())), step
         assert np.array_equal(r.sub_np(), p.sub_np()), step
-    assert r.names() == p.names()
+        reference.pin((reference.hits(r.hits_np()), r.sub_np(), r.cov.value))
+    assert reference.pin(r.names()) == p.names()
     r.sg_gen(), p.sg_gen()
     (ar, sr, ir, _, _), (ap, sp, ip, _, _) = r.graph_np(), p.graph_np()
     assert np.array_equal(canon_arcs(ar), canon_arcs(ap)) and np.array_equal(sr, sp) and np.array_equal(ir, ip)
@@ -102,7 +104,7 @@ def test_port_no_cont(args, hang, frac, ref, port, paf_dir):
     paf = synth.generate(args, f"{paf_dir}/nocont_{len(args)}.paf").encode()
     dr, dp = ref.ma_hit_no_cont(paf, 2000, 100, hang, frac), port.ma_hit_no_cont(paf, 2000, 100, hang, frac)
     names = lambda d: [(d.contents.seq[i].name, d.contents.seq[i].len) for i in range(d.contents.n_seq)]
-    assert names(dr) == names(dp) and (len(names(dr)) > 20 or hang == 4000)
+    assert reference.pin(names(dr)) == names(dp) and (len(names(dr)) > 20 or hang == 4000)
     out = []
     for lib, excl in ((ref, dr), (port, dp)):
         d, n = lib.sd_init(), C.c_size_t(0)
@@ -111,6 +113,7 @@ def test_port_no_cont(args, hang, frac, ref, port, paf_dir):
         out.append((names(d), np.sort(a, order=list(capi.HIT_DT.names))))
         capi.c_free(h), lib.sd_destroy(d)
     assert out[0][0] == out[1][0] and np.array_equal(out[0][1], out[1][1])
+    reference.pin(out[0])
     gone = {nm for nm, _ in names(dr)}
     assert gone and not gone & {nm for nm, _ in out[0][0]}
     ref.sd_destroy(dr), port.sd_destroy(dp)

@@ -9,13 +9,13 @@ import subprocess
 import pytest
 
 from miniasm_b200 import synth
+from tests import reference
 from tests.gfa_compare import assert_same_gfa
 
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CLI = os.path.join(ROOT, "miniasm_b200", "miniasm-b200")
-REF = os.path.join(ROOT, "oracle", "_ref", "miniasm_ref")
 
 SETS = {
     "chaos": "chaos",
@@ -38,19 +38,15 @@ def pafs(built, paf_dir):
     return {k: synth.generate(v, f"{paf_dir}/sw_{k}.paf") for k, v in SETS.items()}
 
 
-@pytest.fixture(scope="module")
-def want(pafs):
-    out = {}
-    for k, path in pafs.items():
-        r = subprocess.run([REF, path], stdout=subprocess.PIPE, stderr=subprocess.PIPE)
-        assert r.returncode == 0
-        out[k] = r.stdout
-    return out
-
-
 @pytest.mark.parametrize("name", list(SETS))
 @pytest.mark.parametrize("env", SWITCHES, ids=lambda e: "+".join(f"{k}={v}" for k, v in e.items()) or "default")
-def test_switch(env, name, pafs, want):
+def test_switch(env, name, pafs):
     r = subprocess.run([CLI, pafs[name]], stdout=subprocess.PIPE, stderr=subprocess.PIPE, env={**os.environ, **env})
     assert r.returncode == 0, r.stderr.decode()[-2000:]
-    assert_same_gfa(r.stdout, want[name], tie_order_free=name in TIES)
+    want = reference.cli([pafs[name]])
+    if want is not None:
+        assert want[0] == 0
+        assert_same_gfa(r.stdout, want[1], tie_order_free=name in TIES)
+    # the digest carries the comparison where the reference is not built; for tied sets only as the sorted line multiset
+    reference.match((r.returncode, r.stdout, r.stderr), [pafs[name]],
+                    lambda x: (x[0], sorted(x[1].split(b"\n")) if name in TIES else x[1]))
